@@ -6,6 +6,7 @@
     python bench.py --config sintel ...                           # configs[2]: 448x1024 (436x1024 padded), iters_pred=24
     python bench.py --config train ...                            # configs[3]: training step 384x512, iters=12
     python bench.py --impl reference --steps K --warmup W         # the reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR                        # also write the last timed step's outputs as DIR/<name>.npy
 
 N > 1 is launched by torchrun (one rank per GPU): the batch axis shards (weak scaling: 4 pairs per GPU); inference has
 no data-path collective, the training step all-reduces one flat gradient buffer (NCCL) and the context encoder's
@@ -49,11 +50,30 @@ UPDATE_LAYERS_N_CHUNKS = ((256, 6), (128, 2), (192, 36), (64, 18), (128, 36), (2
                           (256, 18), (32, 36))
 MASK_MAC_PER_PX = 294_912 + 147_456               # mask[0] 3x3 128->256 + mask[2] 1x1 256->576 (update.py:137-141): only
                                                   # executed on iterations whose prediction is upsampled
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def log(msg):
     """progress on stderr (stdout carries only the JSON line)"""
     print(f'[bench {time.strftime("%H:%M:%S")}] {msg}', file=sys.stderr, flush=True)
+
+
+def dump_outputs(path, arrays):
+    """Write {name: array} as path/<name>.npy: what the last timed step returned to its caller, so that two builds run with
+    the same arguments (hence the same seeded inputs) can be compared output for output.  Tensors keep float32, host scalars
+    become float64.  The largest output (sintel: 4 x 448 x 1024 x 2 float32, 14.7 MB) is stored whole."""
+    import numpy as np
+    out = {}
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a, dtype=np.float64)
+        out[name] = a.astype(np.float64 if a.dtype == np.float64 else np.float32, copy=False)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f'--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES} byte limit')
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + '.npy'), a)
+    log(f'outputs of the last timed step written to {path}: ' + ', '.join(f'{k} {tuple(a.shape)}' for k, a in out.items()))
 
 
 def host_cores():
@@ -157,13 +177,14 @@ def oracle_train_time(cfg, n_pairs, steps, warmup):
         loss.backward()
         torch.nn.utils.clip_grad_norm_([leaves[k] for k in names], 1.0)
         opt.step()
+        return loss.detach()
     for _ in range(warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(steps):
-        step()
+        loss = step()
     dt = time.perf_counter() - t0
-    return n_pairs * steps / dt, dt / steps, cores
+    return n_pairs * steps / dt, dt / steps, cores, loss
 
 
 def run_reference(args, cfg):
@@ -171,11 +192,15 @@ def run_reference(args, cfg):
     if rank != 0:
         return None
     if cfg['train']:
-        pps, sec, cores = oracle_train_time(cfg, 1, args.steps, args.warmup)
+        pps, sec, cores, loss = oracle_train_time(cfg, 1, args.steps, args.warmup)
         what = 'training step (forward + autograd backward + clip + AdamW)'
+        outputs = {'loss': float(loss)}
     else:
-        pps, sec, cores, _ = oracle_forward_time(cfg, 1, args.steps, args.warmup)
+        pps, sec, cores, flow = oracle_forward_time(cfg, 1, args.steps, args.warmup)
         what = 'forward'
+        outputs = {'flow': flow}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     sample = (f'1 pair per step ({cfg["H"]}x{cfg["W"]}, {cfg["iters"]} iterations, {what}), {args.steps} steps after '
               f'{args.warmup} warm-up')
     return {
@@ -247,9 +272,12 @@ def run_ours(args, cfg):
     if train:
         return run_train(args, cfg, model, host, dev_in, timed, barrier, rank, world, local, device)
 
+    last = {}
+
     def step_resident(i):
         a, b = dev_in[i % n_rot]
-        return model([a, b], training=False, last_only=True)[-1]
+        last['flow'] = model([a, b], training=False, last_only=True)[-1]
+        return last['flow']
 
     def step_e2e(i):
         a, b = host[i % n_rot]
@@ -272,6 +300,8 @@ def run_ours(args, cfg):
         sampler.start()
     dev_s, _ = timed(step_resident, args.steps)
     clocks = sampler.stop() if sampler else None
+    # the CUDA graph returns a static buffer that the next replay overwrites: keep the last timed step's flow now
+    timed_flow = last['flow'].cpu() if args.dump_outputs and rank == 0 else None
     launches = launches_per_step * args.steps
     value = world * B * args.steps / dev_s
 
@@ -457,6 +487,8 @@ def run_ours(args, cfg):
                              'sample': f'1 pair ({H}x{W}, {ITERS} iterations) x 3 steps after 1 warm-up, '
                                        'oracle/raft_torch.py on all host cores'},
         }
+    if timed_flow is not None:
+        dump_outputs(args.dump_outputs, {'flow': timed_flow})
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -480,11 +512,13 @@ def run_train(args, cfg, model, host, dev_in, timed, barrier, rank, world, local
     model.compile(optimizer=AdamW(weight_decay=1e-5, learning_rate=sched), clip_norm=1.0)   # :87-98
 
     losses = []
+    last = {}
 
     def step_resident(i):
         a, b = dev_in[i % n_rot]
         out = model.train_step((a, b, dev_fl[i % n_rot], dev_va))
         losses.append(out['loss'])
+        last['metrics'] = out
 
     def step_e2e(i):
         a, b = host[i % n_rot]
@@ -505,6 +539,7 @@ def run_train(args, cfg, model, host, dev_in, timed, barrier, rank, world, local
         sampler.start()
     dev_s, _ = timed(step_resident, args.steps)
     clocks = sampler.stop() if sampler else None
+    timed_metrics = last['metrics']                # what train_step returned on the last timed step: the running metrics
     value = world * B * args.steps / dev_s
     log(f'resident: {value:.2f} pairs/s; end-to-end steps')
     _, e2e_wall = timed(step_e2e, args.steps)
@@ -526,7 +561,7 @@ def run_train(args, cfg, model, host, dev_in, timed, barrier, rank, world, local
         cpu = None
         if not args.quick and world == 1:
             log('CPU baseline: one oracle training step')
-            cpu_pps, _, cores = oracle_train_time(cfg, 1, 1, 0)
+            cpu_pps, _, cores, _ = oracle_train_time(cfg, 1, 1, 0)
             cpu = {'value': cpu_pps, 'unit': 'pairs/s', 'cores': cores, 'kind': 'port',
                    'sample': f'1 pair ({H}x{W}, {ITERS} iterations), one training step of oracle/raft_torch.py under torch.autograd'}
         line = {
@@ -547,6 +582,8 @@ def run_train(args, cfg, model, host, dev_in, timed, barrier, rank, world, local
             'clocks': clocks,
             'cpu_baseline': cpu,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, timed_metrics)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -566,7 +603,11 @@ def main():
                     help='end-to-end leg as one synchronous predict_step per step instead of parallel.predict_stream')
     ap.add_argument('--quick', action='store_true', help='timing only: skip the parity and CPU-baseline legs (A/B runs)')
     ap.add_argument('--precision', default=os.environ.get('RAFT_B200_PRECISION', 'f16x2'), choices=['f16x2', 'fp32'])
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one returned as DIR/<name>.npy (float32 / float64)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     cfg = CONFIGS[args.config]
     # stdout must carry exactly one JSON line: libraries (NCCL prints its version banner there) get stderr instead
     real_stdout = os.dup(1)

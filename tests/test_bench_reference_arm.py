@@ -5,12 +5,15 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), '..'))
 
 
-def test_reference_arm_prints_the_contract_line():
+def test_reference_arm_prints_the_contract_line(tmp_path):
     res = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--impl', 'reference', '--gpus', '1', '--steps', '1',
-                          '--warmup', '1'], capture_output=True, text=True, timeout=900, cwd=ROOT)
+                          '--warmup', '1', '--dump-outputs', str(tmp_path / 'out')], capture_output=True, text=True, timeout=900,
+                         cwd=ROOT)
     assert res.returncode == 0, res.stderr[-2000:]
     lines = [l for l in res.stdout.splitlines() if l.startswith('{')]
     assert len(lines) == 1, res.stdout[-2000:]                       # exactly ONE JSON line
@@ -25,3 +28,7 @@ def test_reference_arm_prints_the_contract_line():
     cb = d['cpu_baseline']
     assert cb['kind'] == 'port' and cb['cores'] >= 1 and cb['value'] == d['value'] and 'pair' in cb['sample']
     assert d['e2e'] == {'value': d['value'], 'unit': 'pairs/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}
+    # --dump-outputs: the final flow of the timed step, one pair at 448x512
+    assert os.listdir(tmp_path / 'out') == ['flow.npy']
+    flow = np.load(tmp_path / 'out' / 'flow.npy')
+    assert flow.dtype == np.float32 and flow.shape == (1, 448, 512, 2) and np.isfinite(flow).all() and np.abs(flow).max() > 0
