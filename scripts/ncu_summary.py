@@ -5,7 +5,7 @@
   python scripts/ncu_summary.py launches.csv --forward [K]    breakdown of the K-th model forward (default: the last
                                                               one whose lookup grid is the largest, i.e. a full batch):
                                                               before-the-loop vs one loop iteration, encoder conv list
-A forward starts at an `image_norm_kernel` pair (feature + context encoder) and ends before the next one.
+A forward starts at a `stem_gather_kernel` pair (feature + context encoder) and ends before the next one.
 """
 import collections, csv, sys
 
@@ -43,7 +43,7 @@ def totals(seq):
 
 
 def forward(seq, which):
-    starts = [i for i, (k, _, _) in enumerate(seq) if k.startswith('image_norm_kernel')]
+    starts = [i for i, (k, _, _) in enumerate(seq) if k.startswith('stem_gather_kernel')]
     fws = []
     for a in range(0, len(starts) - 1, 2):
         end = starts[a + 2] if a + 2 < len(starts) else len(seq)
@@ -51,7 +51,7 @@ def forward(seq, which):
         lk = [int(g.strip('()').split(',')[0]) for k, g, _ in fw if k.startswith('corr_lookup')]
         fws.append((fw, lk[0] if lk else 0))
     if not fws:
-        sys.exit('no forward found (no image_norm_kernel launches)')
+        sys.exit('no forward found (no stem_gather_kernel launches)')
     if which is None:
         big = max(g for _, g in fws)
         which = max(i for i, (fw, g) in enumerate(fws) if g == big and len(fw) == min(len(f) for f, gg in fws if gg == big))

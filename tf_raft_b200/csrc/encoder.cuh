@@ -202,7 +202,7 @@ inline int enc_norm_apply(const EncCtx& c, const EncNormSlot& ns, const float* y
   const float* beta = reinterpret_cast<const float*>(c.prep + ns.beta);
   // (Finalisation inside norm_stats_kernel by the last block of a group was measured twice -- +33 us per launch: the merge
   //  of C channels by one block is serial where norm_final_kernel spreads it over G*C warps; profiles/README.md.)
-  norm_stats_kernel<<<dim3((unsigned)G, kNormSplit), 256, 0, c.st>>>(y, Pg, C, kNormSplit, c.W.part);
+  norm_stats_kernel<<<dim3((unsigned)G, kNormSplit), kNormStatsThreads, 0, c.st>>>(y, Pg, C, kNormSplit, c.W.part);
   norm_final_kernel<<<ceil_div(G * C * 32, 256), 256, 0, c.st>>>(c.W.part, G, C, kNormSplit, gamma, 1e-3f, c.W.mean, c.W.mult);
   norm_apply_kernel<<<grid_for(npix * (pad64(C) / 8)), 256, 0, c.st>>>(y, npix, P, C, c.per_image, c.W.mean, c.W.mult, beta, relu,
                                                                  skip32, skip_hi, skip_lo, out32, hi, lo, pad64(C));
@@ -304,15 +304,8 @@ inline int encoder_forward(int variant, int norm_type, int out_dim, const void* 
   {
     const size_t npix = (size_t)N * h * w;
     const int tot_h = (h - 1) * 2 + 7 - H, tot_w = (w - 1) * 2 + 7 - W;
-    const float* src = images;
-    if (image_norm) {                                 // normalise once (O32 is free until the first ResBlock finishes)
-      const size_t nimg = (size_t)N * H * W * 3;
-      image_norm_kernel<<<grid_for(nimg), 256, 0, st>>>(images, E.O32, nimg);
-      ++g_launches;
-      src = E.O32;
-    }
-    stem_im2col_kernel<<<grid_for(npix * 24), 256, 0, st>>>(src, N, H, W, h, w, (tot_h > 0 ? tot_h : 0) / 2,
-                                                            (tot_w > 0 ? tot_w : 0) / 2, 0, E.Ih, E.Il);
+    stem_gather_kernel<<<dim3(ceil_div(w, kStemSeg), h, N), 256, 0, st>>>(images, H, W, h, w, (tot_h > 0 ? tot_h : 0) / 2,
+                                                                          (tot_w > 0 ? tot_w : 0) / 2, image_norm, E.Ih, E.Il);
     ++g_launches;
     if (!c.stats && pad64(S.c0) != S.c0) {
       RAFT_CUDA_TRY(cudaMemsetAsync(E.Xh, 0, npix * pad64(S.c0) * 2, st));

@@ -537,34 +537,66 @@ __device__ __forceinline__ void chan_merge(float& na, float& ma, float& m2a, flo
   m2a = m2a + m2b + d * d * (na * nb / n);
   na = n;
 }
-__global__ void __launch_bounds__(256) norm_stats_kernel(const float* __restrict__ y, int P, int C, int nsplit,
-                                                         float* __restrict__ part) {
+// Block (g, split) covers pixels [p0, p1) of group g, per = ceil(P / nsplit).  Within it, lanes = 256 / C pixel lanes
+// (lane pl takes pixels p0 + pl, p0 + pl + lanes, ...) and every (lane, channel) sequence is accumulated in pixel order.
+// A thread owns one lane and 4 consecutive channels (C % 4 == 0): float4 loads, kNormStatsAhead pixels of its sequence
+// loaded before they are summed, so that ~16 MB are in flight over the GPU at G = 8 (the scalar one-channel form kept
+// 4 loads per thread in flight and ran latency-bound at ~2.6 TB/s).  The sums, their order and the merge are per channel
+// exactly those of a one-thread-per-(lane, channel) loop, so `part` does not depend on this layout.
+constexpr int kNormStatsThreads = 64;    // = lanes * C / 4 for C dividing 256 (48 of them work at C = 96)
+constexpr int kNormStatsAhead = 32;
+__global__ void __launch_bounds__(kNormStatsThreads) norm_stats_kernel(const float* __restrict__ y, int P, int C,
+                                                                       int nsplit, float* __restrict__ part) {
   __shared__ float red[3][256];
   const int g = blockIdx.x, sp = blockIdx.y;
-  const int lanes = 256 / C > 0 ? 256 / C : 1;          // pixel lanes per block (C <= 256)
-  const int c = threadIdx.x % C, pl = threadIdx.x / C;
+  const int lanes = 256 / C > 0 ? 256 / C : 1;          // pixel lanes per split (C <= 256)
+  const int cq = C / 4;
+  const int c = (threadIdx.x % cq) * 4, pl = threadIdx.x / cq;
   const int per = (P + nsplit - 1) / nsplit;
   const int p0 = sp * per, p1 = min(P, p0 + per);
-  float n = 0.f, mean = 0.f, m2 = 0.f;
+  float n = 0.f, mean[4] = {0.f, 0.f, 0.f, 0.f}, m2[4] = {0.f, 0.f, 0.f, 0.f};
   if (pl < lanes && p0 + pl < p1) {
-    const float* base = y + ((size_t)g * P) * C + c;
-    const float K = base[(size_t)(p0 + pl) * C];
-    float s1 = 0.f, s2 = 0.f;
-    for (int px = p0 + pl; px < p1; px += lanes) {
-      const float v = base[(size_t)px * C] - K;
-      s1 += v;
-      s2 += v * v;
-      n += 1.f;
+    const float4* q = reinterpret_cast<const float4*>(y + ((size_t)g * P + p0 + pl) * C + c);
+    const size_t step = (size_t)lanes * cq;             // float4s from one sample of the sequence to the next
+    const int cnt = (p1 - p0 - pl + lanes - 1) / lanes;
+    const float4 k4 = __ldg(q);                         // shift = the first sample
+    const float K[4] = {k4.x, k4.y, k4.z, k4.w};
+    float s1[4] = {0.f, 0.f, 0.f, 0.f}, s2[4] = {0.f, 0.f, 0.f, 0.f};
+    for (int i = 0; i < cnt; i += kNormStatsAhead) {
+      float4 b[kNormStatsAhead];
+#pragma unroll
+      for (int u = 0; u < kNormStatsAhead; ++u)
+        if (i + u < cnt) b[u] = __ldg(q + (size_t)(i + u) * step);
+#pragma unroll
+      for (int u = 0; u < kNormStatsAhead; ++u) {
+        if (i + u < cnt) {
+          const float x[4] = {b[u].x, b[u].y, b[u].z, b[u].w};
+#pragma unroll
+          for (int e = 0; e < 4; ++e) {
+            const float v = x[e] - K[e];
+            s1[e] += v;
+            s2[e] = __fmaf_rn(v, v, s2[e]);             // s2 += v * v, one rounding (FFMA)
+          }
+          n += 1.f;
+        }
+      }
     }
-    mean = K + s1 / n;
-    m2 = fmaxf(s2 - s1 * s1 / n, 0.f);
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      mean[e] = K[e] + s1[e] / n;
+      m2[e] = fmaxf(s2[e] - s1[e] * s1[e] / n, 0.f);
+    }
   }
-  red[0][threadIdx.x] = n; red[1][threadIdx.x] = mean; red[2][threadIdx.x] = m2;
+  if (pl < lanes) {
+#pragma unroll
+    for (int e = 0; e < 4; ++e) { red[0][pl * C + c + e] = n; red[1][pl * C + c + e] = mean[e]; red[2][pl * C + c + e] = m2[e]; }
+  }
   __syncthreads();
-  if (pl == 0) {
-    for (int l = 1; l < lanes; ++l) chan_merge(n, mean, m2, red[0][l * C + c], red[1][l * C + c], red[2][l * C + c]);
-    float* o = part + (((size_t)g * nsplit + sp) * 3) * C + c;
-    o[0] = n; o[C] = mean; o[2 * C] = m2;
+  for (int ch = threadIdx.x; ch < C; ch += kNormStatsThreads) {     // merge lanes 1..lanes-1 into lane 0, in order
+    float nn = red[0][ch], mm = red[1][ch], mq = red[2][ch];
+    for (int l = 1; l < lanes; ++l) chan_merge(nn, mm, mq, red[0][l * C + ch], red[1][l * C + ch], red[2][l * C + ch]);
+    float* o = part + (((size_t)g * nsplit + sp) * 3) * C + ch;
+    o[0] = nn; o[C] = mm; o[2 * C] = mq;
   }
 }
 // mean[g][c] and mult[g][c] = rsqrt(var + eps) * gamma[c]  (the multiplier applied to (y - mean)).
@@ -654,47 +686,70 @@ __global__ void norm_apply_kernel(const float* __restrict__ y, size_t npix, int 
     }
   }
 }
-// model.py:70-71: x -> 2*(x/255)-1, elementwise (each input value is normalised once here instead of once per
-// 7x7 window position in the im2col gather).
-__global__ void image_norm_kernel(const float* __restrict__ img, float* __restrict__ out, size_t n) {
-  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
-    out[i] = __fsub_rn(__fmul_rn(2.0f, __fdiv_rn(img[i], 255.0f)), 1.0f);
-}
-
-// Stem im2col (extractor.py:95, model.py:70-71): for every output pixel of the 7x7 stride-2 'same' convolution,
-// the 147 input values (tap-major, then rgb) of its window, normalised 2*(x/255)-1, zero outside the image
+// Stem gather (extractor.py:95, model.py:70-71): for every output pixel of the 7x7 stride-2 'same' convolution,
+// the 147 input values (tap-major, then rgb) of its window, optionally normalised 2*(x/255)-1, zero outside the image
 // (padding applies to the normalised image), as fp16 hi/lo planes with 192 channels (147..191 = 0).
-__global__ void stem_im2col_kernel(const float* __restrict__ img, int N, int H, int W, int h, int w, int pad_t,
-                                   int pad_l, int image_norm, __half* __restrict__ hi, __half* __restrict__ lo) {
-  // one thread = 8 consecutive im2col channels of one output pixel -> one 16-byte store per plane
-  const size_t total = (size_t)N * h * w * 24;
-  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-    const int grp = (int)(i % 24);
-    const size_t px = i / 24;
-    const int x = (int)(px % w), y = (int)((px / w) % h), n = (int)(px / ((size_t)w * h));
+// A block owns kStemSeg output pixels of one output row.  It first stages the 7 input rows x (2 * kStemSeg + 5) columns
+// x rgb its windows cover in shared memory (coalesced, each input value loaded and normalised once per block), then
+// writes the planes with one 16-byte store per thread and plane (8 consecutive channels of one pixel).
+constexpr int kStemSeg = 128;
+constexpr int kStemRow = 3 * (2 * kStemSeg + 5);     // floats of one staged input row
+__global__ void __launch_bounds__(256) stem_gather_kernel(const float* __restrict__ img, int H, int W, int h, int w,
+                                                          int pad_t, int pad_l, int image_norm, __half* __restrict__ hi,
+                                                          __half* __restrict__ lo) {
+  __shared__ float tile[7 * kStemRow];
+  const int x0 = blockIdx.x * kStemSeg, y = blockIdx.y, n = blockIdx.z;
+  const int iy0 = 2 * y - pad_t, ix0 = 2 * x0 - pad_l;
+  // tile[ty][3 * (ix - ix0) + rgb]: input row iy0 + ty is contiguous in NHWC from column ix0 on
+  constexpr int kPerRow = (kStemRow + 255) / 256;
+  float v[7][kPerRow];
+#pragma unroll
+  for (int ty = 0; ty < 7; ++ty) {
+    const int iy = iy0 + ty;
+    const float* row = img + (((ptrdiff_t)n * H + iy) * W + ix0) * 3;   // only dereferenced in bounds
+#pragma unroll
+    for (int k = 0; k < kPerRow; ++k) {
+      const int j = threadIdx.x + 256 * k, ix = ix0 + j / 3;
+      v[ty][k] = 0.f;
+      if (j < kStemRow && iy >= 0 && iy < H && ix >= 0 && ix < W) v[ty][k] = __ldg(row + j);
+    }
+  }
+#pragma unroll
+  for (int ty = 0; ty < 7; ++ty) {
+    const int iy = iy0 + ty;
+#pragma unroll
+    for (int k = 0; k < kPerRow; ++k) {
+      const int j = threadIdx.x + 256 * k, ix = ix0 + j / 3;
+      if (j < kStemRow) {
+        float x = v[ty][k];
+        if (image_norm && iy >= 0 && iy < H && ix >= 0 && ix < W) x = __fsub_rn(__fmul_rn(2.0f, __fdiv_rn(x, 255.0f)), 1.0f);
+        tile[ty * kStemRow + j] = x;
+      }
+    }
+  }
+  __syncthreads();
+  const int npx = min(kStemSeg, w - x0);
+  uint4* ohi = reinterpret_cast<uint4*>(hi) + (((size_t)n * h + y) * w + x0) * 24;
+  uint4* olo = reinterpret_cast<uint4*>(lo) + (((size_t)n * h + y) * w + x0) * 24;
+  for (int i = threadIdx.x; i < npx * 24; i += 256) {
+    const int px = i / 24, grp = i - px * 24;
     uint32_t ph[4] = {0u, 0u, 0u, 0u}, pl[4] = {0u, 0u, 0u, 0u};
     if (grp * 8 < 147) {
-      // channel kk = (window row ty) * 21 + j, and the 21 values j = 3 * (window column) + rgb of one window row are
-      // CONTIGUOUS in the NHWC image: walk (ty, j) incrementally instead of dividing per element.
+      // channel kk = (window row ty) * 21 + j, j = 3 * (window column) + rgb: the window of pixel px starts at column
+      // 2 * px of the tile, so its value is tile[ty][6 * px + j]; walk (ty, j) incrementally.
       int ty = (grp * 8) / 21, j = grp * 8 - ty * 21;
-      const int ix0 = 2 * x - pad_l;
-      const float* base = img + ((size_t)n * H * W + ix0) * 3;      // + iy * W * 3 + j  (only dereferenced in bounds)
-      float v[8];
+      const float* t = tile + 6 * px;
+      float f[8];
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
-        const int iy = 2 * y + ty - pad_t, ix = ix0 + ((j * 11) >> 5);   // j / 3 for j < 21
-        v[e] = 0.f;
-        if (ty < 7 && iy >= 0 && iy < H && ix >= 0 && ix < W) {
-          v[e] = __ldg(base + (ptrdiff_t)iy * W * 3 + j);
-          if (image_norm) v[e] = __fsub_rn(__fmul_rn(2.0f, __fdiv_rn(v[e], 255.0f)), 1.0f);
-        }
+        f[e] = ty < 7 ? t[ty * kStemRow + j] : 0.f;
         if (++j == 21) { j = 0; ++ty; }
       }
 #pragma unroll
-      for (int e = 0; e < 4; ++e) split_f16x2(v[2 * e], v[2 * e + 1], ph[e], pl[e]);
+      for (int e = 0; e < 4; ++e) split_f16x2(f[2 * e], f[2 * e + 1], ph[e], pl[e]);
     }
-    reinterpret_cast<uint4*>(hi)[i] = make_uint4(ph[0], ph[1], ph[2], ph[3]);
-    reinterpret_cast<uint4*>(lo)[i] = make_uint4(pl[0], pl[1], pl[2], pl[3]);
+    ohi[i] = make_uint4(ph[0], ph[1], ph[2], ph[3]);
+    olo[i] = make_uint4(pl[0], pl[1], pl[2], pl[3]);
   }
 }
 
