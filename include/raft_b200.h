@@ -237,7 +237,9 @@ int raft_b200_upflow8(const float* flow, int B, int h, int w, float* out, void* 
  *   pyr          : the CorrBlock pyramid (levels entries)
  *   net          : (B,h,w,hidden) in/out -- the tanh() half of cnet's output on entry
  *   inp          : (B,h,w,context)       -- the relu() half
- *   coords1      : (B,h,w,2) in/out; must hold coords_grid(B,h,w) on entry (model.py:89)
+ *   coords1      : (B,h,w,2) in/out; the starting point: coords_grid(B,h,w) (model.py:89), or
+ *                  coords_grid + an initial flow to warm-start the loop (flow is always taken as
+ *                  coords1 - the pixel grid, whatever coords1 held on entry)
  *   flow_up      : iters pointers to (B,8h,8w,2) outputs; entries may be NULL to skip that
  *                  iteration's upsampling (predict_step keeps only the last, model.py:166);
  *                  for BASIC a skipped iteration also skips the mask head.                        */
@@ -245,6 +247,17 @@ int raft_b200_forward_loop(int variant, const void* prepared, const float* const
                            float* net, const float* inp, float* coords1, float* const flow_up[], int iters,
                            int B, int h, int w, void* workspace, size_t workspace_bytes, int precision,
                            void* stream);
+
+/* Warm start for the next pair of a video (the original RAFT's forward_interpolate).
+ * flow (B,h,w,2). Sample (x,y) lands at px = x + fx, py = y + fy (in fp64). It is kept iff
+ * 0 < px < w and 0 < py < h, strictly; NaN is never kept. For every grid point q = (qx,qy):
+ *   out(q) = flow of the kept sample with the least d2 = ((qx-x)-fx)^2 + ((qy-y)-fy)^2,
+ *   evaluated in fp64 op by op (no FMA contraction). Ties go to the lowest row-major index.
+ *   If an image keeps no sample, out = 0 for that image.
+ * out_coords = 1 writes coords_grid + that flow instead (fp32 add): the coords1 the forward loop starts from.
+ * out must not overlap flow (RAFT_ERR_BAD_ARG); B <= 65535, h*w <= 2^30. Cost is O((h*w)^2) per image.
+ * No workspace, no allocation, no sync.                                                           */
+int raft_b200_forward_interpolate(const float* flow, int B, int h, int w, int out_coords, float* out, void* stream);
 
 /* Number of kernels the most recent call on this host thread launched (bench.py's gpu_launches). */
 long long raft_b200_launch_count(void);

@@ -92,6 +92,7 @@ _SIGNATURES = {
     'raft_b200_conv2d': (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i, _i, _vp]),
     'raft_b200_forward_loop': (_i, [_i, _vp, ctypes.POINTER(_vp), _i, _i, _vp, _vp, _vp, ctypes.POINTER(_vp), _i,
                                     _i, _i, _i, _vp, _sz, _i, _vp]),
+    'raft_b200_forward_interpolate': (_i, [_vp, _i, _i, _i, _i, _vp, _vp]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

@@ -776,6 +776,19 @@ int raft_b200_upflow8(const float* flow, int B, int h, int w, float* out, void* 
   return raft_launch_status();
 }
 
+int raft_b200_forward_interpolate(const float* flow, int B, int h, int w, int out_coords, float* out, void* stream) {
+  if (!flow || !out) return RAFT_ERR_BAD_ARG;
+  RAFT_TRY(check_dims(B, h, w));
+  if (B > 65535 || (long long)h * w > (1ll << 30)) return RAFT_ERR_BAD_SHAPE;         // grid.y; int sample indices
+  const size_t n = (size_t)B * h * w * 2;
+  if (out < flow + n && flow < out + n) return RAFT_ERR_BAD_ARG;                      // out must not overlap flow
+  const dim3 grid((unsigned)((h * w + kFwdInterpThreads - 1) / kFwdInterpThreads), (unsigned)B);
+  forward_interpolate_kernel<<<grid, kFwdInterpThreads, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+      flow, h, w, out_coords, out);
+  RAFT_COUNT_LAUNCH();
+  return raft_launch_status();
+}
+
 int raft_b200_encoder_prepared_bytes(int variant, int out_dim, size_t* bytes) {
   if (!bytes || (variant != RAFT_VARIANT_BASIC && variant != RAFT_VARIANT_SMALL)) return RAFT_ERR_BAD_ARG;
   if (out_dim < 32 || out_dim > 256 || out_dim % 32) return RAFT_ERR_BAD_SHAPE;

@@ -826,6 +826,71 @@ __global__ void context_split_kernel(const float* __restrict__ cnet, size_t npix
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Warm start for the next pair of a video (the original RAFT's forward_interpolate): forward-splat
+// the flow of one pair and fill every grid point from the nearest splatted sample.
+//   Sample i = (x, y) lands at (x + fx, y + fy) (fp64) and is kept iff it lands strictly inside
+//   (0, w) x (0, h); NaN never is.  Query q takes the flow of the kept sample with the least
+//   d2 = ((qx-x)-fx)^2 + ((qy-y)-fy)^2, every operation an individually rounded fp64 op, ties to the
+//   lowest sample index (strict < over samples scanned in index order); no kept sample -> 0.
+// Exact brute force, O((h*w)^2) per image: one thread per query, grid (query blocks, B); the block
+// stages the image's samples through shared memory in tiles.  A dropped sample is staged with a NaN
+// flow, so its d2 is NaN and never compares below the running best.
+// ------------------------------------------------------------------------------------------------
+constexpr int kFwdInterpThreads = 128;
+__global__ void __launch_bounds__(kFwdInterpThreads) forward_interpolate_kernel(const float* __restrict__ flow, int h,
+                                                                               int w, int out_coords,
+                                                                               float* __restrict__ out) {
+  __shared__ double2 s_x[kFwdInterpThreads];           // (x, fx)
+  __shared__ double2 s_y[kFwdInterpThreads];           // (y, fy)
+  const int n = h * w;
+  const float* f = flow + (size_t)blockIdx.y * n * 2;
+  const int q = blockIdx.x * kFwdInterpThreads + threadIdx.x;
+  const double qx = (double)(q % w), qy = (double)(q / w);
+  double best = __longlong_as_double(0x7ff0000000000000ll);   // +inf
+  int best_i = -1;
+  for (int t0 = 0; t0 < n; t0 += kFwdInterpThreads) {
+    const int i = t0 + threadIdx.x;
+    if (i < n) {
+      const double x = (double)(i % w), y = (double)(i / w);
+      const double fx = (double)f[2 * i], fy = (double)f[2 * i + 1];
+      const double px = __dadd_rn(x, fx), py = __dadd_rn(y, fy);
+      const bool keep = px > 0.0 && px < (double)w && py > 0.0 && py < (double)h;
+      s_x[threadIdx.x] = make_double2(x, keep ? fx : __longlong_as_double(0x7ff8000000000000ll));
+      s_y[threadIdx.x] = make_double2(y, fy);
+    }
+    __syncthreads();
+    if (q < n) {
+      const int m = min(kFwdInterpThreads, n - t0);
+#pragma unroll 4
+      for (int j = 0; j < m; ++j) {
+        const double2 a = s_x[j], b = s_y[j];
+        const double dx = __dsub_rn(__dsub_rn(qx, a.x), a.y);
+        const double dy = __dsub_rn(__dsub_rn(qy, b.x), b.y);
+        const double d2 = __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy));
+        if (d2 < best) {
+          best = d2;
+          best_i = t0 + j;
+        }
+      }
+    }
+    __syncthreads();
+  }
+  if (q >= n) return;
+  float vx = 0.0f, vy = 0.0f;
+  if (best_i >= 0) {
+    vx = f[2 * best_i];
+    vy = f[2 * best_i + 1];
+  }
+  if (out_coords) {                                    // coords_grid + flow: the coords1 the forward loop starts from
+    vx = __fadd_rn((float)(q % w), vx);
+    vy = __fadd_rn((float)(q / w), vy);
+  }
+  float* o = out + ((size_t)blockIdx.y * n + q) * 2;
+  o[0] = vx;
+  o[1] = vy;
+}
+
 inline int grid_for(size_t n, int block = 256, int cap = kNumSMs * 16) {
   size_t g = (n + block - 1) / block;
   if (g < 1) g = 1;

@@ -17,6 +17,12 @@ from .layers.update import BasicUpdateBlock, SmallUpdateBlock
 from .losses import end_point_error, sequence_loss
 
 
+def _check_image_size(H, W):
+    if H % 8 or W % 8:
+        raise ValueError(f'image height and width must be multiples of 8 (got {H}x{W}); the reference fails in '
+                         'update.py:146 for other sizes -- crop-or-pad first (datasets/dataset.py:323-334)')
+
+
 class RAFT:
     _variant = _lib.VARIANT_BASIC
 
@@ -94,14 +100,19 @@ class RAFT:
         # model.py:70-71 (2*(x/255)-1) happens inside the encoders' first load (raw_image=True)
         fmap1, fmap2 = self.fnet([image1, image2], training=training, raw_image=True)     # :74
         cnet = self.cnet(image1, training=training, raw_image=True)                       # :82
+        net, inp = self._split_context(cnet)
+        return fmap1, fmap2, net, inp
+
+    def _split_context(self, cnet):
+        """model.py:84-86: net = tanh(cnet[..., :hidden]), inp = relu(cnet[..., hidden:]) into fresh buffers."""
         b, h, w, _ = cnet.shape
         net = torch.empty((b, h, w, self.hidden_dim), dtype=torch.float32, device=cnet.device)
         inp = torch.empty((b, h, w, self.context_dim), dtype=torch.float32, device=cnet.device)
-        with torch.cuda.device(cnet.device):                                              # :84-86
+        with torch.cuda.device(cnet.device):
             _lib.check(_lib.lib().raft_b200_context_split(_lib.ptr(cnet), b * h * w, self.hidden_dim,
                                                           self.context_dim, _lib.ptr(net), _lib.ptr(inp),
                                                           _lib.stream()), 'context_split')
-        return fmap1, fmap2, net, inp
+        return net, inp
 
     def _loop(self, corr_block, net, inp, coords1, flow_ups, b, h, w):
         ub = self.update_block
@@ -112,58 +123,88 @@ class RAFT:
                 self.corr_radius, _lib.ptr(net), _lib.ptr(inp), _lib.ptr(coords1), _lib.ptr_array(flow_ups),
                 len(flow_ups), b, h, w, _lib.ptr(ws), ws.numel(), self.precision, _lib.stream()), 'forward_loop')
 
-    def __call__(self, inputs, training, *, last_only=False):
+    def __call__(self, inputs, training, *, last_only=False, flow_init=None):
         """inputs = [image1, image2], each (B, H, W, 3) float in 0..255 on the GPU.
 
         `training` is required, as in the reference (model.py:68).  `last_only=True` (keyword-only
         extra) computes just the final prediction -- what predict_step returns (model.py:166).
+        `flow_init` (keyword-only extra): a (B, H/8, W/8, 2) float32 flow on the model's device; the loop then
+        starts from coords1 = coords_grid + flow_init instead of coords_grid (the original RAFT's warm start
+        for video, see `forward_interpolate` / `VideoFlow`).
         With `use_graph=True` the whole forward of a given input shape is captured once into a CUDA graph
         and replayed; the returned tensors are then static buffers that the next call overwrites."""
         image1, image2 = inputs
         image1, image2 = _lib.f32c(image1), _lib.f32c(image2)
+        if flow_init is not None:
+            flow_init = self._check_flow_init(flow_init, image1.shape)
         self._sync_trained_params()
         if self.use_graph and not training:
-            return self._graph_call(image1, image2, last_only)
-        return self._forward(image1, image2, training, last_only)
+            return self._graph_call(image1, image2, last_only, flow_init)
+        return self._forward(image1, image2, training, last_only, flow_init)
 
-    def _graph_call(self, image1, image2, last_only):
-        key = (tuple(image1.shape), bool(last_only))
+    def _check_flow_init(self, flow_init, image_shape):
+        if not isinstance(flow_init, torch.Tensor):
+            raise ValueError(f'flow_init must be a torch tensor, got {type(flow_init).__name__}')
+        dev = self.device
+        if dev.type == 'cuda' and dev.index is None:
+            dev = torch.device('cuda', torch.cuda.current_device())
+        if flow_init.device != dev:
+            raise ValueError(f'flow_init must be on the model\'s device {dev}, got {flow_init.device}')
+        bs, H, W, _ = image_shape
+        want = (bs, H // 8, W // 8, 2)
+        if tuple(flow_init.shape) != want:
+            raise ValueError(f'flow_init: expected shape {want} for {H}x{W} images, got {tuple(flow_init.shape)}')
+        if flow_init.dtype != torch.float32:
+            raise ValueError(f'flow_init must be float32, got {flow_init.dtype}')
+        return flow_init.contiguous()
+
+    def _graph_call(self, image1, image2, last_only, flow_init=None):
+        key = (tuple(image1.shape), bool(last_only), flow_init is not None)
         entry = self._graphs.get(key)
         if entry is None:
             s1, s2 = image1.clone(), image2.clone()
+            sf = None if flow_init is None else flow_init.clone()
             side = torch.cuda.Stream(device=self.device)
             side.wait_stream(torch.cuda.current_stream(self.device))
             with torch.cuda.stream(side):                      # warm-up: allocations, attributes, weight packing
                 for _ in range(2):
-                    self._forward(s1, s2, False, last_only)
+                    self._forward(s1, s2, False, last_only, sf)
             torch.cuda.current_stream(self.device).wait_stream(side)
             torch.cuda.synchronize(self.device)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                outs = self._forward(s1, s2, False, last_only)
+                outs = self._forward(s1, s2, False, last_only, sf)
             # The captured kernels hold raw addresses of the encoder / update-block workspaces; those caches keep one
             # shape at a time, so the graph entry owns references to the buffers it was captured with.
             keep = [list(m._ws.values()) for m in (self.fnet, self.cnet, self.update_block)]
-            entry = (graph, s1, s2, outs, self._last, keep)
+            entry = (graph, s1, s2, sf, outs, self._last, keep)
             self._graphs[key] = entry
-        graph, s1, s2, outs, last, _keep = entry
+        graph, s1, s2, sf, outs, last, _keep = entry
         s1.copy_(image1, non_blocking=True)
         s2.copy_(image2, non_blocking=True)
+        if sf is not None:
+            sf.copy_(flow_init, non_blocking=True)
         graph.replay()
         self._last = last
         return outs
 
-    def _forward(self, image1, image2, training, last_only):
+    def _forward(self, image1, image2, training, last_only, flow_init=None):
         bs, H, W, _ = image1.shape
-        if H % 8 or W % 8:
-            raise ValueError(f'image height and width must be multiples of 8 (got {H}x{W}); the reference fails in '
-                             'update.py:146 for other sizes -- crop-or-pad first (datasets/dataset.py:323-334)')
-        h, w = H // 8, W // 8
-        iters = self.iters if training else self.iters_pred                  # model.py:92
+        _check_image_size(H, W)
         fmap1, fmap2, net, inp = self._encode(image1, image2, training)
+        coords1 = coords_grid(bs, H // 8, W // 8, self.device)                # :89
+        if flow_init is not None:
+            coords1.add_(flow_init)
+        return self._decode(fmap1, fmap2, net, inp, coords1, training, last_only)
+
+    def _decode(self, fmap1, fmap2, net, inp, coords1, training, last_only):
+        """Everything after the encoders: the correlation pyramid of (fmap1, fmap2) and the iteration loop from
+        `coords1` (updated in place), with `net` / `inp` the split context of image1."""
+        bs, h, w, _ = coords1.shape
+        H, W = 8 * h, 8 * w
+        iters = self.iters if training else self.iters_pred                  # model.py:92
         corr_block = CorrBlock(fmap1, fmap2, num_levels=self.corr_levels, radius=self.corr_radius,
                                precision=self.precision)                      # :77-79
-        coords1 = coords_grid(bs, h, w, self.device)                          # :89
         preds = [torch.empty((bs, H, W, 2), dtype=torch.float32, device=self.device)
                  if (not last_only or i == iters - 1) else None for i in range(iters)]
         if iters:
